@@ -4,6 +4,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (CUDA path)
     python bench.py --impl reference --gpus N --steps K ...  # reference path on the host CPUs
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results as DIR/*.npy
 
 Workload (``config.workload``): the 8-rank data-parallel job of BASELINE configs[1] --
 torchvision resnet18(num_classes=10) in bf16, batch 64 per rank, SGD lr 1e-4, synthetic
@@ -42,6 +43,7 @@ if str(ROOT) not in sys.path:
 WORLD = 8
 BATCH = 64
 METRIC = "cifar_resnet18_train_samples_per_sec"
+DUMP_ELEMS = 1 << 22          # per dumped array: 16 MB of float32, so that a dump stays below 64 MB
 
 
 def parse():
@@ -62,7 +64,16 @@ def parse():
                     help="capture the step with distrib.overlap(model): gradient buckets leave during backward (measured slower "
                          "for this latency-bound step, see profiles/README.md; default: one sync_model launch after backward)")
     ap.add_argument("--no-parity", action="store_true", help="skip the pre-timing parity check against the oracle")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32): loss (every rank), and "
+                         "rank 0's grads (as sync_model averaged them), buffers and params (after optim.step()); "
+                         f"arrays above {DUMP_ELEMS} elements are a fixed seeded sample of that many")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs needs --impl native")
+    return args
 
 
 # =========================================================================== reference arm
@@ -231,12 +242,11 @@ class Replica:
         if self.graph is not None:
             self.graph.replay()
         else:
+            self.optim.zero_grad()                                    # first, so the step's gradients outlive it
             self.loss.copy_(self._fwd_bwd().detach())
         if not (self.overlap and self.graph is not None):
             self.distrib.sync_model(self.model)
         self.optim.step()
-        if self.graph is None:
-            self.optim.zero_grad()
         if e2e:
             return self.loss.item()                                   # device -> host read of the step's result
         return None
@@ -250,6 +260,28 @@ def bf16_ulp_distance(a, b) -> int:
         bits = t.contiguous().view(torch.int16).to(torch.int32) & 0xFFFF
         return torch.where(bits >= 0x8000, 0x8000 - bits, bits)
     return int((key(a) - key(b)).abs().max()) if a.numel() else 0
+
+
+def write_outputs(out_dir: str, snapshot: dict, proc_world: int, proc_rank: int) -> None:
+    """``out_dir/<name>.npy`` in float32 for every array of ``snapshot``; ``loss`` gathers every process's
+    ranks in rank order.  An array longer than DUMP_ELEMS is cut to the same seeded sample of positions
+    on every run, so that two builds can be compared element for element."""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+    arrays = {name: t.float().cpu() for name, t in snapshot.items()}
+    if proc_world > 1:
+        losses = [None] * proc_world
+        dist.all_gather_object(losses, arrays["loss"])
+        arrays["loss"] = torch.cat(losses)
+    if proc_rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        if t.numel() > DUMP_ELEMS:
+            keep = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_ELEMS]
+            t = t[keep.sort().values]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.numpy())
 
 
 def native_arm(args) -> None:
@@ -384,6 +416,16 @@ def native_arm(args) -> None:
     if cuprof:
         torch.cuda.synchronize()
         torch.cuda.profiler.stop()
+    # what the last timed step handed its caller, copied on the device before later steps overwrite it
+    snapshot = None
+    if args.dump_outputs:
+        snapshot = {"loss": torch.stack([rep.loss for rep in replicas])}
+        if proc_rank == 0:
+            model0 = replicas[0].model
+            snapshot["grads"] = torch.cat([p.grad.flatten() for p in model0.parameters()])
+            snapshot["buffers"] = torch.cat([b.flatten() for b in model0.buffers() if b.dtype.is_floating_point])
+            snapshot["params"] = torch.cat([p.detach().flatten() for p in model0.parameters()])
+        torch.cuda.synchronize()
     # kernels of this library inside the timed region: host-side launches plus the ones each graph replay re-issues
     launches = eng.native_launches() - launches0 + args.steps * sum(rep.launches_per_replay for rep in replicas)
     # ---- timed: K steps end to end (H2D batch + D2H loss inside the region)
@@ -399,6 +441,8 @@ def native_arm(args) -> None:
     clocks = sampler.stop() if sampler else None
     if clocks is not None:
         clocks["sampled_over_ms"] = t_load
+    if snapshot is not None:
+        write_outputs(args.dump_outputs, snapshot, proc_world, proc_rank)
 
     # ---- the dominant kernel of this repo, timed live: the whole gradient+buffer bucket of one sync_model call as
     # ONE launch (backward overlap switched off), CUDA events around every launch on its launch stream

@@ -10,7 +10,7 @@ scaled up: student / teacher / adversary MLPs of ``depth`` x ``dim`` x ``dim`` l
     adv_gen = adv(estimate); (mse + adv_gen).backward(); distrib.sync_model(model); optim.step()
 so two models are synchronised per step over one communicator (eager hooks for the adversary, the bucketed
 ``sync_model`` for the generator).  ``AdversarialLoss`` is the UNMODIFIED reference class from
-``baseline/_ref`` (``flashy/adversarial.py:22-89``) running over ``flashy_b200.distrib``; ``dora`` /
+``oracle/_ref`` (``flashy/adversarial.py:22-89``) running over ``flashy_b200.distrib``; ``dora`` /
 ``colorlog`` come from the test-only stand-ins in ``tests/shims``.  Prints one JSON line (rank 0):
 samples/s, ms per step (CUDA events, max over ranks), launches of this library per step.
 """
@@ -25,7 +25,7 @@ from pathlib import Path
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "tests" / "shims"))
-sys.path.append(str(ROOT / "baseline" / "_ref"))
+sys.path.append(str(ROOT / "oracle" / "_ref"))
 
 import torch                      # noqa: E402
 import torch.distributed as dist  # noqa: E402

@@ -22,9 +22,11 @@ def free_port() -> int:
         return s.getsockname()[1]
 
 
-def _entry(rank: int, world: int, port: int, module: str, func: str, args: tuple, backend: str):
+def _entry(rank: int, world: int, port: int, module: str, func: str, args: tuple, backend: str, hide_gpus: bool):
     os.environ.update(RANK=str(rank), LOCAL_RANK=str(rank), WORLD_SIZE=str(world),
                       MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
+    if hide_gpus:
+        os.environ["CUDA_VISIBLE_DEVICES"] = ""
     if str(ROOT) not in sys.path:
         sys.path.insert(0, str(ROOT))
     import torch
@@ -42,11 +44,13 @@ def _entry(rank: int, world: int, port: int, module: str, func: str, args: tuple
             dist.destroy_process_group()
 
 
-def run_ranks(world: int, module: str, func: str, args: tuple = (), backend: str = "gloo", timeout: float = 180.0):
-    """Run ``module.func(rank, world, *args)`` on ``world`` processes; raise if any fails."""
+def run_ranks(world: int, module: str, func: str, args: tuple = (), backend: str = "gloo", timeout: float = 180.0,
+              hide_gpus: bool = False):
+    """Run ``module.func(rank, world, *args)`` on ``world`` processes; raise if any fails.
+    ``hide_gpus``: the processes see no CUDA device, as on a CPU-only machine, whatever this one has."""
     ctx = mp.get_context("spawn")
     port = free_port()
-    procs = [ctx.Process(target=_entry, args=(r, world, port, module, func, args, backend))
+    procs = [ctx.Process(target=_entry, args=(r, world, port, module, func, args, backend, hide_gpus))
              for r in range(world)]
     for p in procs:
         p.start()

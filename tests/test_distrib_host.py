@@ -73,7 +73,7 @@ def _worker(rank, world):
 
 @pytest.mark.parametrize("world", (2, 8))
 def test_distrib_host_logic_gloo(world):
-    run_ranks(world, "tests.test_distrib_host", "_worker")
+    run_ranks(world, "tests.test_distrib_host", "_worker", hide_gpus=True)
 
 
 def test_single_process_is_a_noop():
@@ -101,10 +101,14 @@ def test_single_process_is_a_noop():
 
 def test_virtual_ranks_host_logic():
     """Virtual ranks (threads of one process) see a world of their own; rendezvous works."""
+    run_ranks(1, "tests.test_distrib_host", "_virtual_ranks_worker", backend="none", hide_gpus=True)
+
+
+def _virtual_ranks_worker(proc_rank, proc_world):
     from flashy_b200 import VirtualWorld, distrib
     world = 4
     vw = VirtualWorld(world)
-    assert vw.engine.host_only          # no GPU in this test environment
+    assert vw.engine.host_only          # this process sees no CUDA device
 
     def body(rank, w):
         assert (distrib.rank(), distrib.world_size()) == (rank, w) and w == world

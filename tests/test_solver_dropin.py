@@ -1,6 +1,6 @@
 """A real Flashy solver on the ``flashy_b200`` path.
 
-The UNMODIFIED reference package (``baseline/_ref/flashy``, installed by ``baseline/install_ref.py``:
+The UNMODIFIED reference package (``oracle/_ref/flashy``, installed by ``oracle/install_ref.py``:
 ``BaseSolver`` / ``run_stage`` / ``commit`` / ``restore`` of ``flashy/solver.py:30-211``, ``StateManager``,
 ``AdversarialLoss`` of ``flashy/adversarial.py:22-89``, the logger stack) is imported with
 ``flashy.distrib`` aliased to ``flashy_b200.distrib`` exactly as INTEGRATION.md section 1 shows; ``dora``
@@ -12,7 +12,6 @@ CPU part (W = 1): BASELINE configs[0] -- stages, metric history, checkpoints, re
 GPU part: the CIFAR-style step and ``AdversarialLoss.train_adv`` on 4 virtual ranks, compared with
 the oracle (per-rank gradients averaged by ``oracle/numeric.py``, then the same optimizer step).
 """
-import importlib.util
 import sys
 from argparse import Namespace
 from pathlib import Path
@@ -23,23 +22,18 @@ from torch import nn
 from torch.nn import functional as F
 
 ROOT = Path(__file__).resolve().parent.parent
-REF = ROOT / "baseline" / "_ref"
+REF = ROOT / "oracle" / "_ref"
 SHIMS = ROOT / "tests" / "shims"
 
 
 @pytest.fixture(scope="module")
 def flashy():
     if not (REF / "flashy" / "solver.py").exists():
-        spec = importlib.util.spec_from_file_location("install_ref", ROOT / "baseline" / "install_ref.py")
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        outcome = mod.install()
-        if not (REF / "flashy" / "solver.py").exists():
-            pytest.skip(f"reference not installed in baseline/_ref ({outcome})")
+        pytest.skip("upstream Flashy is not installed in oracle/_ref (build() installs it from an upstream checkout)")
     if str(SHIMS) not in sys.path:
         sys.path.insert(0, str(SHIMS))
     if str(REF) not in sys.path:
-        sys.path.append(str(REF))          # at the end: baseline/_ref also holds the reference's `tests` package
+        sys.path.append(str(REF))
     import flashy_b200.distrib
     sys.modules["flashy.distrib"] = flashy_b200.distrib          # INTEGRATION.md section 1
     import flashy as pkg
