@@ -150,3 +150,109 @@ def loader_indices(n: int, rank: int, world: int, shuffle: bool) -> tp.List[int]
         reps = -(-pad // len(order))
         order += (order * reps)[:pad]
     return order[rank:total:world]
+
+
+# --------------------------------------------------------------------------- kernel reduction contract
+# The collective kernels (flashy_b200/csrc) reduce W columns elementwise: accumulate in rank order in
+# Acc<T> (fp32 for bf16 / fp16, the dtype itself otherwise), divide once for AVG, round once to the wire
+# dtype.  reduce_op restates that arithmetic so that kernel outputs can be compared bit for bit; the
+# float64 reference and error bound below check the restatement itself against the exact operation.
+SUM, AVG, MAX, MIN, PROD = range(5)          # fx_op values (include/flashy_b200.h)
+
+_ACC = {
+    torch.float32: torch.float32, torch.float64: torch.float64,
+    torch.bfloat16: torch.float32, torch.float16: torch.float32,
+    torch.int32: torch.int32, torch.int64: torch.int64,
+}
+
+# unit roundoff u = 2^-p (p = significand bits incl. the implicit one) and the smallest subnormal
+UNIT_ROUNDOFF = {torch.float64: 2.0 ** -53, torch.float32: 2.0 ** -24, torch.bfloat16: 2.0 ** -8, torch.float16: 2.0 ** -11}
+TINY = {torch.float64: 2.0 ** -1074, torch.float32: 2.0 ** -149, torch.bfloat16: 2.0 ** -133, torch.float16: 2.0 ** -24}
+
+
+def _combine(acc: torch.Tensor, x: torch.Tensor, op: int) -> torch.Tensor:
+    # same selection as combine<OP> in fx_device.cuh: ties (+0 / -0) keep the later rank's value
+    if op in (SUM, AVG):
+        return acc + x
+    if op == MAX:
+        return torch.where(acc > x, acc, x)
+    if op == MIN:
+        return torch.where(acc < x, acc, x)
+    if op == PROD:
+        return acc * x
+    raise ValueError(f"unknown op {op}")
+
+
+def reduce_op(columns: tp.Sequence[torch.Tensor], op: int, acc_dtype: tp.Optional[torch.dtype] = None) -> torch.Tensor:
+    """Elementwise reduction of ``columns`` (rank order) as the kernels compute it: accumulate in
+    ``Acc<T>`` in rank order, for AVG one true division by W, one rounding to the input dtype.
+    ``acc_dtype`` overrides the accumulator (tests use it to model a wrong accumulator width)."""
+    dtype = columns[0].dtype
+    if op == AVG and not dtype.is_floating_point:
+        raise ValueError("AVG is defined for floating-point tensors only")
+    acc_t = acc_dtype or _ACC[dtype]
+    acc = columns[0].to(acc_t)
+    for x in columns[1:]:
+        acc = _combine(acc, x.to(acc_t), op)
+    if op == AVG:
+        # a tensor divisor: torch turns division by a Python scalar into a reciprocal multiply on CUDA
+        acc = torch.div(acc, torch.full_like(acc, len(columns)))
+    return acc.to(dtype)
+
+
+def reduce_op_wire_bf16(columns: tp.Sequence[torch.Tensor], op: int) -> torch.Tensor:
+    """fp32 tensors sent over a bf16 wire (FLASHY_B200_WIRE=bf16): every input is rounded to bf16,
+    reduced as a bf16 bucket (fp32 accumulation, one rounding to bf16) and widened back to fp32."""
+    assert columns[0].dtype == torch.float32
+    return reduce_op([c.to(torch.bfloat16) for c in columns], op).to(torch.float32)
+
+
+def reference64(columns: tp.Sequence[torch.Tensor], op: int) -> torch.Tensor:
+    """float64 reference of the operation, independent of the kernels' accumulation order and
+    width.  SUM / AVG use a compensated (Neumaier) sum, so for inputs of at most 53 significant bits
+    the result is the exact sum rounded to float64 up to a few units of 2^-106 relative."""
+    xs = [c.to(torch.float64) for c in columns]
+    if op in (SUM, AVG):
+        s, comp = xs[0].clone(), torch.zeros_like(xs[0])
+        for x in xs[1:]:
+            t = s + x
+            comp += torch.where(s.abs() >= x.abs(), (s - t) + x, (x - t) + s)
+            s = t
+        s = s + comp
+        return s / len(xs) if op == AVG else s
+    acc = xs[0]
+    for x in xs[1:]:
+        acc = torch.maximum(acc, x) if op == MAX else torch.minimum(acc, x) if op == MIN else acc * x
+    return acc
+
+
+def sum_error_bound(columns: tp.Sequence[torch.Tensor], op: int, out_dtype: tp.Optional[torch.dtype] = None,
+                    acc_dtype: tp.Optional[torch.dtype] = None) -> torch.Tensor:
+    """Largest |out - reference64| a correct SUM / AVG may show, elementwise:
+
+        (W-1) u_acc sum_r |x_r| / d  +  u_acc |ref|  +  u_out |ref|  +  tiny_out  +  u_ref |ref|
+
+    d = W for AVG and 1 for SUM; u is the unit roundoff (2^-24 fp32, 2^-53 fp64, 2^-8 bf16,
+    2^-11 fp16) and tiny_out the smallest subnormal of the output dtype.
+
+    Derivation.  Write S = sum_r x_r and s_k for the accumulator after rank k.  Each of the W-1
+    additions is one rounding, s_k = (s_{k-1} + x_k)(1 + e_k) with |e_k| <= u_acc, so
+    |s_W - S| <= u_acc sum_{k>=2} |s_k| <= (W-1) u_acc sum_r |x_r| to first order (the standard
+    recursive-summation bound; every |s_k| is at most sum_r |x_r|).  Division by d is exact
+    for d = 1 and one more rounding for AVG: u_acc |S/d|.  Rounding to the output dtype adds
+    u_out |S/d|, or at most half a subnormal spacing when the result is below the normal range
+    (tiny_out).  Additions of subnormals are exact, so underflow adds nothing before that.
+    The float64 reference carries one rounding of its own division (u_ref = 2^-53; its
+    compensated sum is exact to second order).  Second-order terms (products of two u) are left
+    out: they are below the first-order slack of sum_{k>=2}|s_k| <= (W-1) sum_r |x_r| for every
+    input these tests use.  The bound is meaningful for finite results only."""
+    dtype = columns[0].dtype
+    out_dtype = out_dtype or dtype
+    acc_dtype = acc_dtype or _ACC[dtype]
+    world = len(columns)
+    d = world if op == AVG else 1
+    u_acc, u_out = UNIT_ROUNDOFF[acc_dtype], UNIT_ROUNDOFF[out_dtype]
+    mag = torch.stack([c.to(torch.float64).abs() for c in columns]).sum(0)
+    ref = reference64(columns, op).abs()
+    return ((world - 1) * u_acc * mag / d + (u_acc if op == AVG else 0.0) * ref + u_out * ref
+            + TINY[out_dtype] + (2.0 ** -53) * ref)

@@ -299,7 +299,9 @@ def test_size_independent_properties_at_full_size():
 @pytest.mark.parametrize("world", (2, 3, 5, 8))
 def test_ragged_unaligned_empty_and_odd_worlds(world):
     """Misaligned views, odd lengths, empty tensors, channels_last, world sizes without a
-    compile-time specialisation (3, 5)."""
+    compile-time specialisation (3, 5).  The lists are small enough for the one-shot kernel, which
+    is asserted; the sharded kernels at these layouts and worlds are covered by
+    tests/test_gpu_kernel_matrix.py."""
     from flashy_b200 import distrib
     shapes = [(0,), (1,), (3,), (17,), (1023,), (2, 3, 5, 7), (40000,)]
 
@@ -347,6 +349,9 @@ def test_ragged_unaligned_empty_and_odd_worlds(world):
     for r in range(world):
         for g_, w_ in zip(got[r], want):
             assert torch.equal(g_.contiguous(), w_.contiguous())
+    numels = tuple(int(np.prod(s)) for s in shapes if np.prod(s)) + (400,)
+    plans = [p.info for p in vworld(world).engine.plans.values() if p.key[1] == numels]
+    assert len(plans) == 2 and all(info.kernel == 1 for info in plans)        # fp32 and bf16: k_one_shot
 
 
 def test_mixed_dtypes_and_bucket_splitting(monkeypatch):
@@ -483,10 +488,12 @@ def test_count_mismatch_raises_on_every_rank_cuda():
 
 @pytest.mark.parametrize("dtype", (torch.bfloat16, torch.float32))
 def test_pipelined_kernel_forced_in_loopback(monkeypatch, dtype):
-    """The warp-role pipelined kernel (default on real multi-GPU buckets) forced on for virtual
-    ranks, with small chunks so that every CTA runs several pipeline stages."""
+    """The warp-role pipelined kernel k_pipe (default on real multi-GPU buckets) forced on for
+    virtual ranks, with small chunks so that every CTA runs several pipeline stages.  The fused
+    kernel is switched off: the planner prefers it whenever it is eligible."""
     from flashy_b200 import VirtualWorld, distrib
     import torchvision
+    monkeypatch.setenv("FLASHY_B200_FUSE", "0")
     monkeypatch.setenv("FLASHY_B200_PIPE", "2")
     monkeypatch.setenv("FLASHY_B200_CHUNK_BYTES", "2048")
     world = 8
@@ -510,6 +517,8 @@ def test_pipelined_kernel_forced_in_loopback(monkeypatch, dtype):
         for r in range(world):
             for g, w_ in zip(got[r], want):
                 assert torch.equal(g, w_)
+        sharded = [p.info for p in vw.engine.plans.values() if p.info.algo == 2]
+        assert sharded and all(info.kernel == 4 and info.chunks > 1 for info in sharded)   # k_pipe<NVLS=false>
     finally:
         vw.close()
 

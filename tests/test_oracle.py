@@ -180,3 +180,156 @@ def test_bench_reference_arm_line():
     assert line["metric"] == "cifar_resnet18_train_samples_per_sec" and line["higher_is_better"] is True
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["cpu_baseline"]["kind"] == "port"
     assert line["cpu_baseline"]["cores"] >= 1 and "gloo" in line["cpu_baseline"]["sample"]
+
+
+# ---- the kernels' reduction contract (oracle/numeric.py reduce_op) against exact arithmetic ----------
+from fractions import Fraction  # noqa: E402
+
+# (significand bits incl. the implicit one, smallest normal exponent, largest exponent)
+_FORMATS = {torch.float64: (53, -1022, 1023), torch.float32: (24, -126, 127),
+            torch.bfloat16: (8, -126, 127), torch.float16: (11, -14, 15)}
+_FLOATS = (torch.float32, torch.float64, torch.bfloat16, torch.float16)
+
+
+def _round(q, dtype):
+    """Exact value q (Fraction, or +-inf) rounded to nearest-even in `dtype`, returned as a Fraction or +-inf."""
+    if not isinstance(q, Fraction):
+        return q
+    if q == 0:
+        return Fraction(0)
+    p, emin, emax = _FORMATS[dtype]
+    a = abs(q)
+    e = a.numerator.bit_length() - a.denominator.bit_length()          # 2^e <= a < 2^(e+2)
+    if a >= Fraction(2) ** (e + 1):
+        e += 1
+    elif a < Fraction(2) ** e:
+        e -= 1
+    quantum = Fraction(2) ** (max(e, emin) - p + 1)
+    r = round(a / quantum) * quantum                                      # Fraction.__round__: ties to even
+    if r >= Fraction(2) ** (emax + 1):
+        return float("inf") if q > 0 else float("-inf")
+    return r if q > 0 else -r
+
+
+def _exact(x: float):
+    return Fraction(x) if np.isfinite(x) else x
+
+
+def _add(a, b):
+    if isinstance(a, float) or isinstance(b, float):
+        return float(a) + float(b)
+    return a + b
+
+
+def _stepwise(cols, op, acc_dtype, out_dtype):
+    """The contract evaluated in exact arithmetic with an explicit rounding after every step."""
+    vals = [_exact(float(v)) for v in cols]
+    acc = _round(vals[0], acc_dtype)
+    for x in vals[1:]:
+        if op in (numeric.SUM, numeric.AVG):
+            acc = _round(_add(acc, x), acc_dtype)
+        elif op == numeric.PROD:
+            acc = _round(acc * x, acc_dtype)
+        elif op == numeric.MAX:
+            acc = acc if acc > x else x
+        else:
+            acc = acc if acc < x else x
+    if op == numeric.AVG:
+        acc = _round(acc / len(vals), acc_dtype)
+    return _round(acc, out_dtype)
+
+
+def _columns(dtype, world, n, seed, op):
+    g = torch.Generator().manual_seed(seed)
+    x = torch.randn(world, n, generator=g, dtype=torch.float64)
+    x *= 2.0 ** (torch.randint(-12, 13, (world, n), generator=g)).double()   # magnitudes 2^+-12 apart
+    if op == numeric.PROD:
+        x = 1 + x / (1 + x.abs()) / 4                                        # stay near 1
+    x[-1, : n // 4] = -x[:-1, : n // 4].sum(0) * (1 + 2.0 ** -7)             # cancellation columns
+    return [c.to(dtype) for c in x]
+
+
+@pytest.mark.parametrize("world", (2, 3, 5, 8))
+@pytest.mark.parametrize("dtype", _FLOATS)
+@pytest.mark.parametrize("op", (numeric.SUM, numeric.AVG, numeric.MAX, numeric.MIN, numeric.PROD))
+def test_reduce_op_equals_stepwise_exact_rounding(world, dtype, op):
+    """reduce_op is the exact result rounded through the kernels' steps; SUM / AVG lie inside the bound."""
+    cols = _columns(dtype, world, 64, 1000 * world + op, op)
+    got = numeric.reduce_op(cols, op)
+    assert got.dtype == dtype
+    acc = numeric._ACC[dtype]
+    bound = numeric.sum_error_bound(cols, op) if op in (numeric.SUM, numeric.AVG) else None
+    ref64 = numeric.reference64(cols, op)
+    for j in range(got.numel()):
+        want = _stepwise([c[j] for c in cols], op, acc, dtype)
+        assert _exact(float(got[j])) == want, (j, float(got[j]), float(want))
+        exact_vals = [Fraction(float(c[j])) for c in cols]
+        if op in (numeric.SUM, numeric.AVG):
+            exact = sum(exact_vals) / (world if op == numeric.AVG else 1)
+            assert abs(Fraction(float(got[j])) - exact) <= Fraction(float(bound[j])), j
+            assert abs(float(got[j]) - float(ref64[j])) <= float(bound[j]), j
+        elif op == numeric.MAX:
+            assert float(ref64[j]) == float(max(exact_vals)) == float(got[j])
+        elif op == numeric.MIN:
+            assert float(ref64[j]) == float(min(exact_vals)) == float(got[j])
+
+
+@pytest.mark.parametrize("world", (2, 3, 8))
+@pytest.mark.parametrize("dtype", (torch.int32, torch.int64))
+@pytest.mark.parametrize("op", (numeric.SUM, numeric.MAX, numeric.MIN, numeric.PROD))
+def test_reduce_op_integers_exact(world, dtype, op):
+    g = torch.Generator().manual_seed(world + 10 * op)
+    hi = 4 if op == numeric.PROD else 1 << 20
+    cols = [torch.randint(-hi, hi, (50,), generator=g, dtype=dtype) for _ in range(world)]
+    if dtype == torch.int64 and op != numeric.PROD:
+        cols = [c + (-1) ** r * (1 << 60) for r, c in enumerate(cols)]          # 64-bit magnitudes
+    got = numeric.reduce_op(cols, op)
+    fold = {numeric.SUM: lambda a, b: a + b, numeric.MAX: max, numeric.MIN: min, numeric.PROD: lambda a, b: a * b}[op]
+    for j in range(50):
+        want = int(cols[0][j])
+        for c in cols[1:]:
+            want = fold(want, int(c[j]))
+        assert int(got[j]) == want
+    with pytest.raises(ValueError):
+        numeric.reduce_op(cols, numeric.AVG)
+
+
+def test_reduce_op_wire_bf16_rounds_inputs_then_reduces_as_bf16():
+    g = torch.Generator().manual_seed(3)
+    cols = [torch.randn(256, generator=g) for _ in range(5)]
+    got = numeric.reduce_op_wire_bf16(cols, numeric.AVG)
+    assert got.dtype == torch.float32
+    for j in range(256):
+        want = _stepwise([c[j].bfloat16() for c in cols], numeric.AVG, torch.float32, torch.bfloat16)
+        assert Fraction(float(got[j])) == want
+    assert not torch.equal(got, numeric.reduce_op(cols, numeric.AVG))         # the wire rounding is visible
+
+
+def test_reduce_op_special_values():
+    inf, nan = float("inf"), float("nan")
+    cols = [torch.tensor([inf, inf, -0.0, nan, 1e-45, 6.0e4]), torch.tensor([1.0, -inf, -0.0, 1.0, 1e-45, 6.0e4])]
+    s = numeric.reduce_op(cols, numeric.SUM)
+    assert s[0] == inf and torch.isnan(s[1]) and torch.isnan(s[3])
+    assert s[2] == 0 and torch.signbit(s[2])                                    # -0 + -0 = -0
+    assert s[4] == 2 * cols[0][4] and s[4] < 2.0 ** -126                        # subnormal sum is exact
+    half = numeric.reduce_op([c.half() for c in cols], numeric.SUM)
+    assert half[5] == inf                                                       # fp16 SUM overflows ...
+    assert numeric.reduce_op([c.half() for c in cols], numeric.AVG)[5] == 6.0e4  # ... its mean does not
+    m = numeric.reduce_op([torch.tensor([0.0]), torch.tensor([-0.0])], numeric.MAX)
+    assert torch.signbit(m[0])                                                  # tie keeps the later rank, as combine<MAX>
+
+
+@pytest.mark.parametrize("dtype,step", ((torch.bfloat16, 2.0 ** -9), (torch.float16, 2.0 ** -12)))
+def test_bound_rejects_16_bit_accumulation(dtype, step):
+    """A mean accumulated in the 16-bit type itself falls outside the bound on cancellation and
+    small-increment inputs, so the bound tells a wrong accumulator width from a right one."""
+    world = 8
+    small = [torch.tensor([1.0, 1.0], dtype=dtype)] + [torch.tensor([step, 2 * step], dtype=dtype)] * (world - 2) \
+        + [torch.tensor([-1.0, -1.0], dtype=dtype)]
+    for op in (numeric.SUM, numeric.AVG):
+        ref = numeric.reference64(small, op)
+        bound = numeric.sum_error_bound(small, op)
+        good = numeric.reduce_op(small, op)
+        assert bool(((good.double() - ref).abs() <= bound).all())
+        bad = numeric.reduce_op(small, op, acc_dtype=dtype)
+        assert bool(((bad.double() - ref).abs() > bound).any()), (op, bad, ref)
